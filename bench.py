@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo (CUDA, sm_100a)
     python bench.py --impl reference --gpus N ...            # the reference's CPU algorithm (oracle)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's results as .npy
 
 A "step" is ONE multi-scalar multiplication of 2^LOG2N uniformly random BN254 scalars against a
 resident commitment key (CE::commit with r = 0, benches/commit.rs:30,112-125).
@@ -287,8 +288,11 @@ def run_b200(args):
     # bases are P_i = (K0 + i) G, so the MSM must equal [sum_i s_i (K0 + i)] G: one scalar-mul on the oracle side
     result_check = None
     if rank == 0:
-        result_check = closed_form_check(args.log2n, (d_out if world > 1 else d_part).cpu().numpy().tobytes(),
-                                         out_host.raw if world == 1 else h_pinned_t.numpy().tobytes())
+        device_result = (d_out if world > 1 else d_part).cpu().numpy().tobytes()
+        e2e_result = out_host.raw if world == 1 else h_pinned_t.numpy().tobytes()
+        result_check = closed_form_check(args.log2n, device_result, e2e_result)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"msm_device": device_result, "commit_e2e": e2e_result})
 
     # ---------------- the same sharded MSM at the other sizes north_star names -------------------
     other_sizes = [time_other_size(lg, steps=5, warmup=3) for lg in args.other_log2n if lg != args.log2n]
@@ -406,6 +410,20 @@ def closed_form_check(log2n, device_result_jac, e2e_result_jac):
     return {"device_result_equals_closed_form": bool(got_dev == exp), "e2e_result_equals_closed_form": bool(got_e2e == exp),
             "ok": bool(got_dev == exp and got_e2e == exp),
             "checker": "oracle: [sum_i s_i (k0+i)] G by one scalar multiplication (bases are (k0+i) G)"}
+
+
+def dump_outputs(out_dir, jacobian_results):
+    """--dump-outputs: every MSM result of the last timed step as DIR/<name>.npy, float32 of shape (2, 32): the affine
+    x and y in canonical (non-Montgomery) form, 32 little-endian bytes each, so every value is exact.  Affine because
+    another build may return the same point with other Jacobian coordinates; the point at infinity is all zeros."""
+    import numpy as np
+
+    from nova_b200.provider import Curve, _jac_to_affine
+    os.makedirs(out_dir, exist_ok=True)
+    for name, jac in jacobian_results.items():
+        point = _jac_to_affine(Curve(CURVE), jac) or (0, 0)
+        raw = b"".join(v.to_bytes(32, "little") for v in point)
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.frombuffer(raw, dtype=np.uint8).reshape(2, 32).astype(np.float32))
 
 
 def effective_cores():
@@ -580,7 +598,7 @@ def run_workload_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 20, or 3 with --workload)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--log2n", type=int, default=20)
@@ -594,14 +612,20 @@ def main():
                     help="N > 1: how the ranks' partial sums are combined (fused = peer stores inside the reduction kernel)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-prove-step", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the MSM results of the last timed step to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 20 if args.workload == "msm" else 3
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.workload != "msm" or args.impl != "b200"):
+        ap.error("--dump-outputs writes the results of the MSM workload on --impl b200 only")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     if args.workload != "msm":
         if args.workload == "hyperkzg" and "--log2n" not in sys.argv:
             args.log2n = 22
-        if "--steps" not in sys.argv:
-            args.steps = 3
         (run_workload_reference if args.impl == "reference" else run_workload)(args)
     elif args.impl == "reference":
         run_reference(args)

@@ -118,11 +118,12 @@ static int sumcheck_mode(const char* path) {
   return 0;
 }
 
-// --concurrency <log2n> [threads]: the same `threads` commitments issued from ONE thread one after the other and from
-// `threads` threads at once (what rayon does in the reference: src/spartan/ppsnark.rs:457-470); the results must be the
-// same points and the ratio of the two wall times is printed.  Synthetic key, pinned host scalars.
+// --concurrency <log2n> <threads> <points.bin>: the same `threads` commitments issued from ONE thread one after the other
+// and from `threads` threads at once (what rayon does in the reference: src/spartan/ppsnark.rs:457-470); the results must
+// be the same points (written to points.bin) and the ratio of the two wall times is printed.  Synthetic key, pinned host
+// scalars.
 #include <chrono>
-static int concurrency_mode(int log2n, int nthreads) {
+static int concurrency_mode(int log2n, int nthreads, const char* points_path) {
   check(b200_init(0), "b200_init");
   const size_t n = (size_t)1 << log2n;
   // generator of BN254 G1 (1, 2) in Montgomery form is not needed here: any valid affine point works as the seed of
@@ -170,12 +171,14 @@ static int concurrency_mode(int log2n, int nthreads) {
   // same points?  compare cross-multiplied (Jacobian coordinates differ between runs): done by the Python side from the dump
   std::printf("{\"what\": \"%d commits of 2^%d scalars, serial vs %d threads\", \"ms_serial\": %.4f, \"ms_concurrent\": %.4f, "
               "\"speedup\": %.3f}\n", nthreads, log2n, nthreads, ms_serial, ms_conc, ms_serial / ms_conc);
-  FILE* f = std::fopen("/tmp/concurrency_points.bin", "wb");
-  if (f) {
-    std::fwrite(serial.data(), sizeof(Point), nthreads, f);
-    std::fwrite(conc.data(), sizeof(Point), nthreads, f);
-    std::fclose(f);
+  FILE* f = std::fopen(points_path, "wb");
+  if (!f) {
+    std::fprintf(stderr, "cannot write %s\n", points_path);
+    return 1;
   }
+  std::fwrite(serial.data(), sizeof(Point), nthreads, f);
+  std::fwrite(conc.data(), sizeof(Point), nthreads, f);
+  std::fclose(f);
   for (void* b : bufs) b200_host_free(b);
   b200_ck_release(ck);
   return 0;
@@ -225,7 +228,7 @@ int main(int argc, char** argv) {
   if (std::string(argv[1]) == "--sumcheck") return argc > 2 ? sumcheck_mode(argv[2]) : 2;
   if (std::string(argv[1]) == "--mgpu") return argc > 3 ? mgpu_mode(argv[2], std::atoi(argv[3])) : 2;
   if (std::string(argv[1]) == "--concurrency")
-    return argc > 2 ? concurrency_mode(std::atoi(argv[2]), argc > 3 ? std::atoi(argv[3]) : 4) : 2;
+    return argc > 4 ? concurrency_mode(std::atoi(argv[2]), std::atoi(argv[3]), argv[4]) : 2;
   std::ifstream f(argv[1], std::ios::binary);
   check(b200_init(0), "b200_init");
   auto bases = rd<Affine>(f);

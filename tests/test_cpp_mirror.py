@@ -226,7 +226,7 @@ def check_sumcheck(exe, oracle, tmp_path):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("log2n", [14, 18])
-def test_cpp_concurrent_commits_overlap_and_agree(log2n):
+def test_cpp_concurrent_commits_overlap_and_agree(log2n, tmp_path):
     """host_mirror_test --concurrency: 4 commitments issued from one thread in turn and from 4 threads at once
     (rayon in the reference: ppsnark.rs:457-470) give the same points; each call takes its own host slot (workspace +
     streams) of the key, so the calls overlap on the device -- the measured ratio is printed (profiles/r02e)."""
@@ -234,9 +234,10 @@ def test_cpp_concurrent_commits_overlap_and_agree(log2n):
 
     from nova_b200.provider import Curve, _jac_to_affine
     build()
-    out = subprocess.check_output([EXE, "--concurrency", str(log2n), "4"], text=True, timeout=300)
+    points = tmp_path / "concurrency_points.bin"
+    out = subprocess.check_output([EXE, "--concurrency", str(log2n), "4", str(points)], text=True, timeout=300)
     res = json.loads(out.strip().splitlines()[-1])
-    raw = open("/tmp/concurrency_points.bin", "rb").read()
+    raw = points.read_bytes()
     pts = [_jac_to_affine(Curve(0), raw[96 * i:96 * i + 96]) for i in range(8)]
     assert pts[:4] == pts[4:] and len(set(pts[:4])) == 4
     assert res["ms_serial"] > 0 and res["ms_concurrent"] > 0
